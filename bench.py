@@ -5,8 +5,10 @@ vs the HBM roofline), one JSON line on stdout.
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload short|tagged|mixed|stable|medium|asm|unstable] [--records R]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU gaf2paf on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's output to DIR/*.npy (see dump_outputs)
 
-A step is one pass of the whole device pipeline (DESIGN.md §4) over one synthetic batch.
+A step is one pass of the whole device pipeline (DESIGN.md §4) over one synthetic batch.  The inputs are generated
+from fixed seeds, so runs with the same arguments convert the same bytes.
 
 * `value`  — the batch already resident in HBM (CUDA events around exactly K steps, max over ranks).
 * `e2e`    — the same metric through the host-buffer C-ABI call g2p_convert_host (pinned host input ->
@@ -22,6 +24,7 @@ and two small all-gathers of sizes).  Per-GPU work is fixed as N grows: "scaling
 """
 import argparse
 import ctypes
+import hashlib
 import json
 import mmap
 import os
@@ -208,6 +211,42 @@ class CpuArm:
         self.td.cleanup()
 
 
+DUMP_WINDOWS, DUMP_WINDOW_BYTES = 128, 64 << 10   # the output text sample: 8 MiB of bytes, 32 MiB as float32
+
+
+def dump_outputs(dirname, g2p, d_out, res, suffix=""):
+    """--dump-outputs: what the timed call returned in its last step, for comparing two builds output for output.
+
+    paf.npy              the output text as byte values (float32): all of it when it fits the sample, else
+                         DUMP_WINDOWS windows of DUMP_WINDOW_BYTES at offsets drawn with a fixed seed
+    paf_offsets.npy      the start offset of each window (float64)
+    paf_byte_counts.npy  how often each byte value 0..255 occurs in the whole output (float64)
+    paf_md5.npy          the 16 bytes of the md5 digest of the whole output (float64): equal only for equal outputs
+    result.npy           n_records, out_bytes, exit code, rec_status, rec_aux, err_record, stage, mid_bytes (float64);
+                         timings and per-kernel record counts are left out, they are not part of the result"""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    n = int(res.out_bytes)
+    if n <= DUMP_WINDOWS * DUMP_WINDOW_BYTES:
+        offsets = np.zeros(1, dtype=np.int64)
+        sample = np.frombuffer(g2p.copy_to_host(d_out, n), dtype=np.uint8)
+    else:
+        offsets = np.sort(np.random.default_rng(0).choice(n - DUMP_WINDOW_BYTES + 1, DUMP_WINDOWS, replace=False))
+        sample = np.concatenate([np.frombuffer(g2p.copy_to_host(d_out + int(o), DUMP_WINDOW_BYTES), dtype=np.uint8) for o in offsets])
+    counts = np.zeros(256, dtype=np.int64)
+    digest = hashlib.md5()
+    chunk = 64 << 20
+    for o in range(0, n, chunk):
+        part = g2p.copy_to_host(d_out + o, min(chunk, n - o))
+        counts += np.bincount(np.frombuffer(part, dtype=np.uint8), minlength=256)
+        digest.update(part)
+    fields = [res.n_records, res.out_bytes, g2p.exit_code(res), res.rec_status, res.rec_aux, res.err_record, res.stage, res.mid_bytes]
+    for name, arr in (("paf", sample.astype(np.float32)), ("paf_offsets", offsets.astype(np.float64)),
+                      ("paf_byte_counts", counts.astype(np.float64)), ("paf_md5", np.frombuffer(digest.digest(), dtype=np.uint8).astype(np.float64)),
+                      ("result", np.array(fields, dtype=np.float64))):
+        np.save(os.path.join(dirname, name + suffix + ".npy"), arr)
+
+
 def run_reference(a):
     """--impl reference: the reference's own CPU implementation on the host cores."""
     import helpers as H
@@ -293,7 +332,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cli", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     if a.impl == "reference":
         return run_reference(a)
@@ -437,6 +479,9 @@ def main():
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     t_ms = max_float(e0.elapsed_time(e1))
+    if a.dump_outputs:
+        # before the e2e calls below, which reuse the converter's output buffer
+        dump_outputs(a.dump_outputs, g2p, d_out, res, "_rank%d" % rank if world > 1 else "")
 
     # ---- end to end through the host-buffer C-ABI call (pinned input, H2D + D2H inside); the per-rank results
     # stay in per-rank pinned buffers whose rank order is the record order (a gather list, what writev consumes)

@@ -4,7 +4,8 @@ or unusual records.  Compares exit code and stdout (and stderr text for rc 1).
 
     python tests/fuzz_vs_ref.py [--n 2000] [--seed 1] [--bin build/g2p_hostsim] [--long]
 
-Development tool (needs oracle/_ref, i.e. the build container).  CIGAR text outside the SAM
+The reference is the unmodified build in oracle/_ref when present, else the restatement
+oracle/bin/gaf2paf_oracle (tests/helpers.py oracle_path).  CIGAR text outside the SAM
 grammar that std::stol accepts is handled like the reference does; the only tolerated class is
 int64 overflow (undefined behaviour in the reference), see `tolerated()`.
 """
@@ -17,7 +18,8 @@ import sys
 import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "gaf2paf")
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import helpers as H  # noqa: E402
 
 LENGTHS = "chrA\t1000\nchrB\t500\nchrC\t300\na\t10\nb\t5\nc\t10\nn2\t20\nn3\t50\nz\t0\naveryveryverylongname_12345\t77\n"
 
@@ -136,6 +138,7 @@ def main():
     ap.add_argument("--long", action="store_true", help="append a 300-byte tag to every case: the records take the long-record kernels (k_par, k_long)")
     a = ap.parse_args()
     rnd = random.Random(a.seed)
+    ref_bin, kind = H.oracle_path()
     bad = 0
     tol = 0
     with tempfile.TemporaryDirectory() as td:
@@ -149,7 +152,7 @@ def main():
             if a.long:
                 data += "\tzy:Z:" + "p" * 300
             data = data.encode("latin-1") + b"\n"
-            ref = run(REF, lp, data)
+            ref = run(ref_bin, lp, data)
             got = run(a.bin, lp, data)
             same = ref[0] == got[0] and (ref[0] == 134 or ref[1] == got[1]) and (ref[0] != 1 or ref[2] == got[2])
             if not same:
@@ -161,7 +164,7 @@ def main():
                     print("MISMATCH #%d: %r" % (it, data))
                     print("   ref rc=%d out=%r err=%r" % (ref[0], ref[1][:200], ref[2][-160:]))
                     print("   got rc=%d out=%r err=%r" % (got[0], got[1][:200], got[2][-160:]))
-    print("fuzz: %d cases, %d mismatches, %d tolerated (int64-overflow UB in the reference)" % (a.n, bad, tol))
+    print("fuzz: %d cases, %d mismatches, %d tolerated (int64-overflow UB in the reference), %s oracle" % (a.n, bad, tol, kind))
     return 1 if bad else 0
 
 

@@ -129,6 +129,23 @@ def golden(name):
         return json.load(f)
 
 
+def reference_cli(tool, args, subst):
+    """(exit code, stdout, stderr) of the reference `tool` on a command line it rejects, its own path written X in stderr:
+    the reference build when present, else the run stored in tests/golden/reference_runs.json.  `args` may hold the
+    placeholders of that file ({L}, {A}, {G}); `subst` maps them to paths."""
+    ref = os.path.join(REF_BIN, tool)
+    if os.path.exists(ref):
+        rc, out, err = run_tool(ref, [subst.get(a, a) for a in args])
+        return rc, out, err.replace(ref, "X")
+    for r in golden("reference_runs.json")["cli"][tool]:
+        if r["args"] == list(args):
+            err = r["err"]
+            for k, v in subst.items():
+                err = err.replace(k, v)
+            return r["rc"], r["out"].encode("latin-1"), err
+    raise KeyError("no stored %s run for %r: add it to tests/golden/make_reference_runs.py" % (tool, args))
+
+
 # ---- gaf2unstable: synthetic rGFA + stable-coordinate GAF (BASELINE config 2 shape) -------------
 def gen_rgfa_case(seed, n_contigs=4, n_records=500, aligned=False, multi_ref_pct=3):
     """Returns (rgfa bytes, gaf bytes).  Rank-0 chains over `n_contigs` reference contigs (one with an

@@ -349,7 +349,7 @@ def test_gaf2unstable_abort_and_cli(g2p):
     rgfa, gaf = H.gen_rgfa_case(21, n_records=1500, aligned=True)
     bad = gaf + b"q\t100\t0\t15\t+\t>nosuchcontig:0-15\t15\t0\t15\t15\t15\t60\tcg:Z:15M\n" + gaf[:2000]
     exe = os.path.join(g2p.BIN_DIR, "gaf2unstable")
-    ref_exe = os.path.join(H.REF_BIN, "gaf2unstable")
+    ref_exe, _kind = H.oracle_path("auto", "gaf2unstable")   # the reference build when present, else the restatement
     with tempfile.TemporaryDirectory() as td:
         gp, a = os.path.join(td, "g.gfa"), os.path.join(td, "a.gaf")
         open(gp, "wb").write(rgfa)
@@ -365,10 +365,11 @@ def test_gaf2unstable_abort_and_cli(g2p):
         assert out == rout[:len(out)]
         assert out.count(b"\n") == sum(1 for ln in gaf.split(b"\n")[:-1] if not ln.startswith(b"*"))   # records before the failing one
         # usage errors
-        for args in ([], [a], [a, "b", "c", "-g", gp]):
-            rc, out, err = H.run_tool(exe, args)
-            rrc, rout, rerr = H.run_tool(ref_exe, args)
-            assert rc == rrc and err.replace(exe, "X") == rerr.replace(ref_exe, "X")
+        subst = {"{A}": a, "{G}": gp}
+        for args in ([], ["{A}"], ["{A}", "b", "c", "-g", "{G}"]):
+            rc, out, err = H.run_tool(exe, [subst.get(x, x) for x in args])
+            rrc, rout, rerr = H.reference_cli("gaf2unstable", args, subst)
+            assert rc == rrc and err.replace(exe, "X") == rerr
 
 
 def test_descriptor_overflow_falls_back_to_reparsing_emit(g2p, monkeypatch):
