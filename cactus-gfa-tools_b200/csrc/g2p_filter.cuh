@@ -57,30 +57,116 @@ struct FilterMeta {
 };
 
 // ---- stof of a tag value (gi:f:0.978): decimal digits, optional fraction and exponent; anything else -> false -----
+// Correctly rounded (to nearest, ties to even) like std::stof, and false where stof throws std::out_of_range: a value that
+// rounds (24 bits, unbounded exponent) to 2^128 or more, or to less than FLT_MIN.  Method: at most 19 significant digits
+// go into an integer M (a non-zero digit beyond them sets `sticky`), value = M * 10^E.  A double estimate gives a 24-bit
+// candidate m * 2^e within one unit of the result; exact comparisons of M * 10^E with the midpoints next to the candidate
+// (288-bit integers) correct it.  When digits were dropped and a midpoint lies between M * 10^E and (M + 1) * 10^E the
+// rounding is not decided by the digits kept: false (more than 19 significant digits within 10^-18 of a midpoint).
+struct FBig { u32 w[9]; };   // 288 bits: M * 10^56 * 2^26 and M * 2^153 fit
+G2P_HD void fbig_set(FBig& a, u64 v) {
+    a.w[0] = (u32)v; a.w[1] = (u32)(v >> 32);
+    for (int i = 2; i < 9; ++i) a.w[i] = 0;
+}
+G2P_HD void fbig_mul(FBig& a, u32 f) {
+    u64 c = 0;
+    for (int i = 0; i < 9; ++i) { const u64 t = (u64)a.w[i] * f + c; a.w[i] = (u32)t; c = t >> 32; }
+}
+G2P_HD void fbig_mul_pow10(FBig& a, u32 k) {
+    for (; k >= 9; k -= 9) fbig_mul(a, 1000000000u);
+    u32 p = 1;
+    while (k--) p *= 10;
+    fbig_mul(a, p);
+}
+G2P_HD void fbig_shl(FBig& a, u32 s) {
+    const u32 ws = s >> 5, bs = s & 31u;
+    for (int i = 8; i >= 0; --i) {
+        const int j = i - (int)ws;
+        const u32 hi = j >= 0 ? a.w[j] : 0u, lo = j >= 1 ? a.w[j - 1] : 0u;
+        a.w[i] = bs ? (hi << bs) | (lo >> (32 - bs)) : hi;
+    }
+}
+// sign of M * 10^E - n * 2^b
+G2P_HD int fdec_cmp(u64 M, i32 E, u64 n, i32 b) {
+    FBig x, y;
+    fbig_set(x, M); fbig_set(y, n);
+    if (E >= 0) fbig_mul_pow10(x, (u32)E); else fbig_mul_pow10(y, (u32)-E);
+    if (b >= 0) fbig_shl(y, (u32)b); else fbig_shl(x, (u32)-b);
+    for (int i = 8; i >= 0; --i) if (x.w[i] != y.w[i]) return x.w[i] < y.w[i] ? -1 : 1;
+    return 0;
+}
+// sign of value - n * 2^b for a value in [M, M + 1) * 10^E (sticky: strictly inside); 2 = not decided
+G2P_HD int fdec_cmp_value(u64 M, bool sticky, i32 E, u64 n, i32 b) {
+    const int c = fdec_cmp(M, E, n, b);
+    if (!sticky || c > 0) return c;
+    if (c == 0) return 1;
+    return fdec_cmp(M + 1, E, n, b) > 0 ? 2 : -1;
+}
 G2P_HD bool parse_float_text(const u8* s, u32 n, float& out) {
     u32 i = 0;
     bool neg = false;
     if (i < n && (s[i] == '+' || s[i] == '-')) { neg = s[i] == '-'; ++i; }
-    double v = 0.0;
-    u32 nd = 0;
-    while (i < n && s[i] >= '0' && s[i] <= '9') { v = v * 10.0 + (s[i] - '0'); ++i; ++nd; }
+    u64 M = 0;
+    u32 nd = 0, sig = 0;
+    i32 E = 0;
+    bool sticky = false;
+    for (; i < n && s[i] >= '0' && s[i] <= '9'; ++i, ++nd) {
+        const u32 d = s[i] - '0';
+        if (sig < 19) { M = M * 10 + d; sig += M != 0; }
+        else { ++E; sticky |= d != 0; }
+    }
     if (i < n && s[i] == '.') {
-        ++i;
-        double scale = 0.1;
-        while (i < n && s[i] >= '0' && s[i] <= '9') { v += (s[i] - '0') * scale; scale *= 0.1; ++i; ++nd; }
+        for (++i; i < n && s[i] >= '0' && s[i] <= '9'; ++i, ++nd) {
+            const u32 d = s[i] - '0';
+            if (sig < 19) { M = M * 10 + d; sig += M != 0; --E; }
+            else sticky |= d != 0;
+        }
     }
     if (nd == 0) return false;
     if (i < n && (s[i] == 'e' || s[i] == 'E')) {
         ++i;
         bool eneg = false;
         if (i < n && (s[i] == '+' || s[i] == '-')) { eneg = s[i] == '-'; ++i; }
-        u32 e = 0, ne = 0;
-        while (i < n && s[i] >= '0' && s[i] <= '9' && ne < 3) { e = e * 10 + (s[i] - '0'); ++i; ++ne; }
+        i32 x = 0;
+        u32 ne = 0;
+        for (; i < n && s[i] >= '0' && s[i] <= '9'; ++i, ++ne) if (x < 100000) x = x * 10 + (s[i] - '0');
         if (ne == 0) return false;
-        for (u32 k = 0; k < e; ++k) v = eneg ? v / 10.0 : v * 10.0;
+        E += eneg ? -x : x;
     }
     if (i != n) return false;   // (stof ignores trailing text; such values are not produced by gaf2paf: unsupported)
-    out = (float)(neg ? -v : v);
+    if (M == 0) { out = neg ? -0.f : 0.f; return true; }
+    if ((i32)sig - 1 + E >= 39) return false;   // >= 10^39: overflow
+    if ((i32)sig + E <= -38) return false;      // < 10^-38: below FLT_MIN
+    // estimate: |E| <= 56 roundings of a double, far below half a unit of the float
+    double v = (double)M;
+    for (i32 k = 0; k < E; ++k) v *= 10.0;
+    for (i32 k = 0; k < -E; ++k) v /= 10.0;
+    union { double d; u64 u; } db;
+    db.d = v;
+    const u64 mant = (db.u & ((1ULL << 52) - 1)) | (1ULL << 52);   // v = mant * 2^(exp - 1075), a normal double
+    u64 m = (mant + (1ULL << 28)) >> 29;
+    i32 e = (i32)((db.u >> 52) & 0x7ff) - 1075 + 29;
+    if (m == (1ULL << 24)) { m >>= 1; ++e; }
+    for (int it = 0; it < 3; ++it) {
+        const int up = fdec_cmp_value(M, sticky, E, 2 * m + 1, e - 1);
+        if (up == 2) return false;
+        if (up > 0 || (up == 0 && (m & 1))) {
+            if (++m == (1ULL << 24)) { m >>= 1; ++e; }
+            continue;
+        }
+        const bool low = m == (1ULL << 23);   // the next float down is half a unit away
+        const int dn = low ? fdec_cmp_value(M, sticky, E, 4 * m - 1, e - 2) : fdec_cmp_value(M, sticky, E, 2 * m - 1, e - 1);
+        if (dn == 2) return false;
+        if (dn < 0 || (dn == 0 && (m & 1))) {
+            if (low) { m = (1ULL << 24) - 1; --e; } else --m;
+            continue;
+        }
+        break;
+    }
+    if (e >= 105 || e < -149) return false;   // >= 2^128, < 2^-126 (stof: std::out_of_range)
+    union { float f; u32 u; } fb;
+    fb.u = (neg ? 0x80000000u : 0u) | ((u32)(e + 150) << 23) | ((u32)m & 0x7FFFFFu);
+    out = fb.f;
     return true;
 }
 

@@ -1,11 +1,12 @@
 #!/usr/bin/env python3
 """Mutation fuzzer for gaffilter: the filter kernels under the SIMT emulator (build/g2p_filter_simt) vs the reference
 gaffilter on small inputs (a few query sequences, ~40 records) with one or two mutated records, random option sets, GAF and
-PAF mode.  Compares the exit code, stdout and the "[gaffilter]: ..." summary line.
+PAF mode.  Compares the exit code, stdout and the "[gaffilter]: ..." summary line.  The checker is the reference build
+(oracle/_ref/gaffilter) when present, else the restatement oracle/bin/gaffilter_oracle (tests/helpers.py oracle_path).
 
     python tests/fuzz_filter_vs_ref.py [--n 1000] [--seed 1]
 
-Development tool (needs oracle/_ref)."""
+Development tool; tests/test_filter_edges.py runs a few hundred of these cases."""
 import argparse
 import os
 import random
@@ -37,7 +38,7 @@ def main():
     ap.add_argument("--seed", type=int, default=1)
     a = ap.parse_args()
     rnd = random.Random(a.seed)
-    ref_bin = os.path.join(H.REF_BIN, "gaffilter")
+    ref_bin, kind = H.oracle_path("auto", "gaffilter")
     bad = 0
     for it in range(a.n):
         paf = rnd.random() < 0.5
@@ -59,7 +60,7 @@ def main():
                     print("     " + repr(l))
                 print("   ref rc=%d lines=%d err=%r" % (ref[0], ref[1].count(b"\n"), ref[2][-120:]))
                 print("   got rc=%d lines=%d err=%r" % (got[0], got[1].count(b"\n"), got[2][-120:]))
-    print("fuzz gaffilter: %d cases, %d mismatches" % (a.n, bad))
+    print("fuzz gaffilter: %d cases, %d mismatches, %s oracle" % (a.n, bad, kind))
     return 1 if bad else 0
 
 

@@ -9,8 +9,8 @@ compare with them, so that those tests also run where the reference build (oracl
   written X and the paths of input files as the placeholders the arguments use ({L} lengths, {A} GAF, {G} graph).
 * "gaffilter": gaffilter on the inputs of tests/test_filter.py's GPU tests (tests/helpers.py gen_filter_case) -- exit
   code, md5 and size of stdout (megabytes: too large to store), stderr.
-* "gaffilter_inputs": every run of tests/test_filter.py's emulator tests (ref_gaffilter), keyed by the md5 of the input
-  and the arguments -- exit code, md5 of stdout, last stderr line.
+* "gaffilter_inputs": gaffilter on tests/test_filter.py stored_inputs(), keyed by the md5 of the input and the
+  arguments -- exit code, md5 of stdout, last stderr line.
 
 --source reference (the default) runs oracle/_ref/<tool> and stops when that build is missing.  --source project
 records this project's executables and its filter kernels under the SIMT emulator (build/g2p_filter_simt) instead:
@@ -20,7 +20,6 @@ import argparse
 import hashlib
 import json
 import os
-import subprocess
 import sys
 import tempfile
 
@@ -94,16 +93,14 @@ def filter_runs(td, source):
 
 
 def emulator_test_runs(source):
-    """Run tests/test_filter.py's emulator tests with ref_gaffilter recording what it compares with."""
-    with tempfile.TemporaryDirectory() as td:
-        rec = os.path.join(td, "runs.jsonl")
-        env = dict(os.environ, G2P_RECORD_GAFFILTER=rec)
-        subprocess.check_call([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "-m", "not gpu", "-k", "emulated",
-                               os.path.join(ROOT, "tests", "test_filter.py")], env=env, cwd=ROOT)
-        runs = {}
-        for line in open(rec):
-            r = json.loads(line)
-            runs[r.pop("key")] = r
+    """gaffilter on the inputs of tests/test_filter.py stored_inputs() (the emulator tests' inputs when this was first
+    recorded; the restatement oracle/bin/gaffilter_oracle must reproduce them)."""
+    import test_filter
+    exe = os.path.join(H.REF_BIN, "gaffilter") if source == "reference" else os.path.join(H.BUILD, "g2p_filter_simt")
+    runs = {}
+    for text, args in test_filter.stored_inputs():
+        rc, out, err = H.run_tool(exe, args + ["-"], text)
+        runs["%s %s" % (hashlib.md5(text).hexdigest(), " ".join(args))] = {"rc": rc, "md5": hashlib.md5(out).hexdigest(), "err": err.strip().split("\n")[-1]}
     return runs
 
 

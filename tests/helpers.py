@@ -92,8 +92,8 @@ def gen_records_into(p, first, count, addr, cap, threads=None):
 
 
 def oracle_path(kind="auto", tool="gaf2paf"):
-    """Path of the checker binary: the unmodified reference build when present
-    (kind 'reference'), else the restatement (kind 'port')."""
+    """Path of the checker binary of `tool` (gaf2paf, gaf2unstable, gaffilter): the unmodified reference build when
+    present (kind 'reference'), else the restatement oracle/bin/<tool>_oracle (kind 'port')."""
     ref = os.path.join(REF_BIN, tool)
     port = os.path.join(ORACLE_BIN, tool + "_oracle")
     if kind in ("auto", "reference") and os.path.exists(ref):
@@ -287,6 +287,25 @@ def gen_filter_case(seed, n_records=3000, n_queries=150, paf=False):
     return paf_text, lengths
 
 
-def run_gaffilter_ref(text, args):
-    binary = os.path.join(REF_BIN, "gaffilter")
-    return run_tool(binary, ["-"] + list(args), text)
+def gen_spread_filter_case(seed, n_records=6000, n_queries=3, depth=4, paf=False):
+    """Like gen_filter_case, but with few query sequences whose records lie along the whole query (assembly contigs mapped
+    in pieces): each record's query interval moves by a random offset, about `depth` records cover a query position."""
+    import random
+    rnd = random.Random(seed)
+    gaf, lengths = gen_filter_case(seed, n_records=n_records, n_queries=n_queries)
+    span = max(1, n_records // n_queries * 120 // depth)
+    out = []
+    for ln in gaf.split(b"\n")[:-1]:
+        f = ln.split(b"\t")
+        if f[0] != b"*":
+            off = rnd.randrange(span)
+            f[1] = b"%d" % (int(f[1]) + span)
+            f[2] = b"%d" % (int(f[2]) + off)
+            f[3] = b"%d" % (int(f[3]) + off)
+        out.append(b"\t".join(f))
+    gaf = b"\n".join(out) + b"\n"
+    if not paf:
+        return gaf
+    rc, paf_text, err, kind = run_gaf2paf_cpu(gaf, lengths)
+    assert rc == 0, err
+    return paf_text
