@@ -41,8 +41,11 @@ $(BUILD)/gafgen: tools/gafgen.cpp
 	@mkdir -p $(BUILD)
 	$(CXX) $(CXXFLAGS) -DGAFGEN_MAIN -pthread -o $@ $<
 
-hostsim: $(BUILD)/g2p_hostsim $(BUILD)/g2p_simt $(BUILD)/g2p_simt_long $(BUILD)/g2u_hostsim $(BUILD)/g2u_simt $(BUILD)/g2u_simt_small $(BUILD)/gaf2paf_stub $(BUILD)/g2p_filter_simt $(BUILD)/g2p_floatparse
+hostsim: $(BUILD)/g2p_hostsim $(BUILD)/g2p_simt $(BUILD)/g2p_simt_long $(BUILD)/g2u_hostsim $(BUILD)/g2u_simt $(BUILD)/g2u_simt_small $(BUILD)/gaf2paf_stub $(BUILD)/g2p_filter_simt $(BUILD)/g2p_filter_job_simt $(BUILD)/g2p_floatparse
 $(BUILD)/g2p_filter_simt: tests/hostsim/g2p_filter_simt.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
+	@mkdir -p $(BUILD)
+	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -Itests/hostsim -o $@ $<
+$(BUILD)/g2p_filter_job_simt: tests/hostsim/g2p_filter_job_simt.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -Itests/hostsim -o $@ $<
 $(BUILD)/g2p_floatparse: tests/hostsim/g2p_floatparse.cpp tests/hostsim/cuda_shim.hpp $(HDRS)

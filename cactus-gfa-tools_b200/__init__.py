@@ -40,6 +40,8 @@ EXPORTED_SYMBOLS = (
     "g2p_load_rgfa", "g2p_rgfa_node_lengths", "g2p_unstable_device", "g2p_unstable_host", "g2p_unstable_warnings", "g2p_format_unstable_warning",
     "g2p_unstable_convert_device", "g2p_unstable_convert_host", "g2p_unstable_convert_warnings",
     "g2p_filter_device", "g2p_filter_host",
+    "g2p_filter_job_create", "g2p_filter_job_load", "g2p_filter_job_decide", "g2p_filter_job_emit", "g2p_filter_job_get_stats",
+    "g2p_filter_job_destroy",
 )
 
 
@@ -86,6 +88,12 @@ class FilterResult(ctypes.Structure):
     _fields_ = [("n_loaded", ctypes.c_uint64), ("n_filtered", ctypes.c_uint64), ("filtered_len", ctypes.c_uint64), ("out_bytes", ctypes.c_uint64),
                 ("rec_status", ctypes.c_uint32), ("gpu_launches", ctypes.c_uint32), ("err_record", ctypes.c_uint64),
                 ("device_ms", ctypes.c_float), ("pad", ctypes.c_uint32)]
+
+
+class FilterJobStats(ctypes.Structure):
+    """struct g2p_filter_job_stats (include/g2p.h)."""
+    _fields_ = [("load_ms", ctypes.c_double), ("decide_ms", ctypes.c_double), ("emit_ms", ctypes.c_double),
+                ("h2d_bytes", ctypes.c_uint64), ("d2h_bytes", ctypes.c_uint64)]
 
 
 class Warn(ctypes.Structure):
@@ -143,6 +151,18 @@ def _load():
     lib.g2p_filter_device.restype = ctypes.c_int
     lib.g2p_filter_host.argtypes = [vp, vp, sz, ctypes.POINTER(FilterParams), ctypes.POINTER(vp), ctypes.POINTER(FilterResult)]
     lib.g2p_filter_host.restype = ctypes.c_int
+    lib.g2p_filter_job_create.argtypes = [ctypes.POINTER(vp), ctypes.c_int, ctypes.POINTER(FilterParams), ctypes.POINTER(vp)]
+    lib.g2p_filter_job_create.restype = ctypes.c_int
+    lib.g2p_filter_job_load.argtypes = [vp, ctypes.c_uint64, vp, sz]
+    lib.g2p_filter_job_load.restype = ctypes.c_int
+    lib.g2p_filter_job_decide.argtypes = [vp, ctypes.POINTER(FilterResult)]
+    lib.g2p_filter_job_decide.restype = ctypes.c_int
+    lib.g2p_filter_job_emit.argtypes = [vp, ctypes.c_uint64, vp, sz, ctypes.POINTER(vp), ctypes.POINTER(FilterResult)]
+    lib.g2p_filter_job_emit.restype = ctypes.c_int
+    lib.g2p_filter_job_get_stats.argtypes = [vp, ctypes.POINTER(FilterJobStats)]
+    lib.g2p_filter_job_get_stats.restype = ctypes.c_int
+    lib.g2p_filter_job_destroy.argtypes = [vp]
+    lib.g2p_filter_job_destroy.restype = None
     lib.g2p_unstable_warnings.argtypes = [vp, ctypes.POINTER(ctypes.POINTER(Warn)), ctypes.POINTER(sz)]
     lib.g2p_unstable_warnings.restype = ctypes.c_int
     lib.g2p_format_unstable_warning.argtypes = [vp, vp, sz, vp, sz]
@@ -327,6 +347,55 @@ class Converter:
         buf = ctypes.create_string_buffer(2048)
         lib.g2p_format_error(ctypes.byref(res), addr, n, buf, len(buf))
         return buf.value.decode("latin-1")
+
+
+class FilterJob:
+    """gaffilter on inputs of any size over one or more :class:`Converter` contexts (g2p_filter_job_*): ``load`` every
+    newline-aligned chunk (numbered from 0 in input order; chunk c runs on converters[c % len(converters)]), ``decide``
+    once (-> the FilterResult of the whole input), then ``emit`` every chunk again (-> its kept records)."""
+
+    def __init__(self, converters, params):
+        self._cvs = list(converters)
+        hs = (ctypes.c_void_p * len(self._cvs))(*[cv._h.value for cv in self._cvs])
+        h = ctypes.c_void_p()
+        self._params = params
+        rc = lib.g2p_filter_job_create(hs, len(self._cvs), ctypes.byref(params), ctypes.byref(h))
+        if rc != G2P_OK:
+            raise G2PError("g2p_filter_job_create failed with %d" % rc)
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            lib.g2p_filter_job_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    def _check(self, rc, chunk=0):
+        if rc != G2P_OK:
+            self._cvs[chunk % len(self._cvs)]._check(rc)
+
+    def load(self, chunk, text):
+        addr, n, keep = _buf_ptr(text)
+        self._check(lib.g2p_filter_job_load(self._h, chunk, addr, n), chunk)
+
+    def decide(self):
+        res = FilterResult()
+        self._check(lib.g2p_filter_job_decide(self._h, ctypes.byref(res)))
+        return res
+
+    def emit(self, chunk, text):
+        """-> (kept records of the chunk, FilterResult of the chunk)."""
+        addr, n, keep = _buf_ptr(text)
+        out = ctypes.c_void_p()
+        res = FilterResult()
+        self._check(lib.g2p_filter_job_emit(self._h, chunk, addr, n, ctypes.byref(out), ctypes.byref(res)), chunk)
+        return _bytes_at(out.value, res.out_bytes), res
+
+    def stats(self):
+        s = FilterJobStats()
+        lib.g2p_filter_job_get_stats(self._h, ctypes.byref(s))
+        return s
 
 
 def copy_to_host(d_ptr, n):

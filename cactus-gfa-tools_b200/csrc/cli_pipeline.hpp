@@ -139,6 +139,7 @@ struct Chunk {
     std::string err_text;      // stderr text that belongs before this chunk's output (gaf2unstable warnings)
     std::string open_error;    // non-empty: not a data chunk -- an input could not be opened (printed in order, then exit 1)
     int state = 0;             // 0 free, 1 filled, 2 converted
+    size_t seq = 0;            // chunk number, in input order
 };
 
 struct Pipeline {
@@ -185,6 +186,7 @@ struct Pipeline {
             };
             auto publish = [&](Chunk& c) {
                 std::lock_guard<std::mutex> g(mu);
+                c.seq = s;
                 c.state = c.open_error.empty() ? 1 : 2;
                 ++s;
                 cv.notify_all();

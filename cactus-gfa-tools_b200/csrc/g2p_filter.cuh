@@ -22,6 +22,9 @@
 // Records are kept in input order.  Anything the reference would die on (assert / uncaught exception) is reported as
 // an abort status with the index of the first such line; nothing is printed then (the reference loads all records
 // before it prints any).
+//
+// Inputs of any size and several GPUs go through the job (g2p_filter_job_*, see the bucket partition below and
+// g2p_filter_job.hpp): the same kernels over newline-aligned chunks, the rows partitioned by query name.
 #pragma once
 #include "g2u_core.cuh"
 
@@ -42,7 +45,9 @@ struct __attribute__((aligned(16))) FRow {
     u32 flags;           // kFRowPrimary, kFRowSkip, kFRowHasGi
     float gi;            // GAF mode: stof(gi) when present
     u32 name_len;
+    u64 grec;            // record number: chunk << 32 | line of the chunk (the single call: the line)
 };
+static_assert(sizeof(FRow) == 96, "FRow is the 96-byte row the filter job keeps in host memory");
 enum : u32 { kFRowPrimary = 1u, kFRowSkip = 2u, kFRowHasGi = 4u };
 
 struct FilterMeta {
@@ -53,7 +58,9 @@ struct FilterMeta {
     u64 filtered_len;    // "total block lengths filtered"
     u64 out_total;
     u32 unsupported;     // a query_start >= 2^32: not sortable here
-    u32 assert_rec;      // smallest record on which an assertion of the reference's filter loop fires (0xFFFFFFFF: none)
+    u32 assert_rec;      // smallest row on which an assertion of the reference's filter loop fires (0xFFFFFFFF: none)
+    u64 assert_grec;     // ... its grec, input order across the chunks and partitions of the job (~0: none); the
+                         // single call's rows are its lines, so there both are the line
 };
 
 // ---- stof of a tag value (gi:f:0.978): decimal digits, optional fraction and exponent; anything else -> false -----
@@ -283,14 +290,23 @@ struct FilterArgs {
     u64* keys;      // [nrec]  hash32 << 32 | query_start   (skipped lines: all ones -> sorted to the end)
     u32* vals;      // [nrec]  record index
     FilterMeta* meta;
+    u64 grec_base;  // chunk << 32 (0 for the single call)
 };
+
+// sort key of a loaded row: hash32 << 32 | query_start
+G2P_HD u64 filter_sort_key(const FRow& row) {
+    const u32 h32 = (u32)(row.h0 ^ (row.h0 >> 32) ^ row.h1 ^ (row.h1 >> 32));
+    // (negative starts -- no real aligner writes them, std::stol reads them -- sort together with start 0: the
+    // forward scan of k_filter_sweep never stops on a start <= 0)
+    return ((u64)(h32 == 0xffffffffu ? 0xfffffffeu : h32) << 32) | (u64)(row.qs < 0 ? 0u : (u32)row.qs);
+}
 
 __global__ void __launch_bounds__(128) k_filter_parse(const FilterArgs a) {
     for (u32 r = blockIdx.x * blockDim.x + threadIdx.x; r < a.nrec; r += gridDim.x * blockDim.x) {
         const u32 s = a.rec_start[r], len = a.rec_start[r + 1] - s - 1;
         FRow row;
         row.h0 = row.h1 = 0; row.qs = row.qe = row.qlen = row.block_length = row.matches = 0; row.rc = 0; row.paf_bases = 0;
-        row.mapq = 0; row.flags = 0; row.gi = 0.f; row.name_len = 0;
+        row.mapq = 0; row.flags = 0; row.gi = 0.f; row.name_len = 0; row.grec = a.grec_base | r;
         u32 st = a.P.is_paf ? filter_parse_paf(a.text + s, len, row) : filter_parse_gaf(a.text + s, len, row);
         u64 key = ~0ULL;
         if ((st & 0xff) == ST_SKIP) row.flags |= kFRowSkip;
@@ -298,10 +314,7 @@ __global__ void __launch_bounds__(128) k_filter_parse(const FilterArgs a) {
         else {
             atomicAdd(&a.meta->n_loaded, 1u);
             if (row.qs > 0xFFFFFFF0LL) atomicExch(&a.meta->unsupported, 1u);
-            const u32 h32 = (u32)(row.h0 ^ (row.h0 >> 32) ^ row.h1 ^ (row.h1 >> 32));
-            // (negative starts -- no real aligner writes them, std::stol reads them -- sort together with start 0: the
-            // forward scan of k_filter_sweep never stops on a start <= 0)
-            key = ((u64)(h32 == 0xffffffffu ? 0xfffffffeu : h32) << 32) | (u64)(row.qs < 0 ? 0u : (u32)row.qs);
+            key = filter_sort_key(row);
         }
         a.rows[r] = row;
         a.keys[r] = key;
@@ -552,13 +565,48 @@ __global__ void __launch_bounds__(128) k_filter_sweep(const u64* __restrict__ ke
             filter_interval(rj, lo, hi);
             if (hi >= qstart && lo <= qstop) { const bool d = filter_pair_ok(ri, rj, P, boom); ok = ok && d; }
         }
-        if (boom) atomicMin(&meta->assert_rec, i);
+        if (boom) {   // (local row order is not input order across the job's buckets: grec is)
+            atomicMin(&meta->assert_rec, i);
+            atomicMin(reinterpret_cast<unsigned long long*>(&meta->assert_grec), (unsigned long long)rows[i].grec);
+        }
         keep[i] = ok ? 1 : 0;
         if (!ok) {
             atomicAdd(&meta->n_filtered, 1u);
             atomicAdd(reinterpret_cast<unsigned long long*>(&meta->filtered_len), (unsigned long long)(P.is_paf ? ri.paf_bases : ri.block_length));
         }
     }
+}
+
+// ---- the job (inputs of any size, several GPUs): rows partitioned by query-name bucket -----------------------------
+// Whether a record is kept depends only on the records with the same query name, so the rows of a chunk are
+// partitioned by bucket = the top 8 bits of the name's hash32 and every range of buckets is decided on its own.
+// Load pass: k_filter_bucket_key, 3 radix passes (stable: input order within a bucket, unloaded lines last),
+// k_filter_bucket_offsets, k_filter_gather_rows -> the chunk layout.  Decide pass: k_filter_rekey over the rows of a
+// range of buckets, then the sort, k_filter_ends / k_segmax and k_filter_sweep.  Emit pass: k_filter_scatter_keep.
+constexpr u32 kFBuckets = 256;
+__global__ void __launch_bounds__(128) k_filter_bucket_key(const u64* __restrict__ keys, u32 n, u64* __restrict__ pkeys) {
+    for (u32 r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += gridDim.x * blockDim.x)
+        pkeys[r] = keys[r] == ~0ULL ? (u64)kFBuckets : keys[r] >> 56;
+}
+// off[b] = first position whose bucket is >= b (b = 0 .. kFBuckets; off[kFBuckets] = loaded rows), over sorted pkeys
+__global__ void __launch_bounds__(128) k_filter_bucket_offsets(const u64* __restrict__ pkeys, u32 n, u32* __restrict__ off) {
+    for (u32 p = blockIdx.x * blockDim.x + threadIdx.x; p <= n; p += gridDim.x * blockDim.x) {
+        const u32 lo = p == 0 ? 0u : (u32)pkeys[p - 1] + 1u;
+        const u32 hi = p == n ? kFBuckets : (u32)pkeys[p];
+        for (u32 b = lo; b <= hi && b <= kFBuckets; ++b) off[b] = p;
+    }
+}
+__global__ void __launch_bounds__(128) k_filter_gather_rows(const FRow* __restrict__ rows, const u32* __restrict__ vals, u32 n, FRow* __restrict__ out) {
+    for (u32 p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) out[p] = rows[vals[p]];
+}
+__global__ void __launch_bounds__(128) k_filter_rekey(const FRow* __restrict__ rows, u32 n, u64* __restrict__ keys, u32* __restrict__ vals) {
+    for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        keys[i] = filter_sort_key(rows[i]);
+        vals[i] = i;
+    }
+}
+__global__ void __launch_bounds__(128) k_filter_scatter_keep(const u32* __restrict__ vals, const u8* __restrict__ keep_layout, u32 n, u8* __restrict__ keep) {
+    for (u32 p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) keep[vals[p]] = keep_layout[p];
 }
 
 // ---- printing a kept record ---------------------------------------------------------------------------

@@ -188,6 +188,33 @@ typedef struct g2p_filter_result {
 int g2p_filter_device(g2p_ctx* ctx, const void* d_text, size_t n, const g2p_filter_params* params, void** d_out, g2p_filter_result* res, void* stream);
 int g2p_filter_host(g2p_ctx* ctx, const char* text, size_t n, const g2p_filter_params* params, const char** out, g2p_filter_result* res);
 
+/* gaffilter on inputs of any size and on several GPUs.  Whether a record is kept depends only on the records with the
+ * same query name, so the job partitions the rows by query name (256 buckets of the name hash) and decides each range of
+ * buckets on its own, on any context.  Three passes over the same newline-aligned chunks (each < 4 GiB, numbered from 0
+ * in input order; chunk c runs on ctxs[c % nctx]):
+ *   load    (every chunk)  parse; the loaded rows, in bucket order, go to host memory (~97 B per record in all)
+ *   decide  (once)         the totals and the status of the whole input, as g2p_filter_host reports them for it: a line
+ *                          that fails to load wins (its global line number), then a query_start >= 2^32 (G2P_E_ARG, the
+ *                          same message), then a filter-loop assertion (the smallest global line); nothing may be
+ *                          printed unless rec_status is 0.  G2P_E_TOOBIG when one bucket alone has more records than a
+ *                          GPU can sort (a single query with ~10^9 alignments).  Uses one host thread per context.
+ *   emit    (every chunk)  the kept records of the chunk, printed like g2p_filter_host prints them; the chunk must be
+ *                          the one loaded (bytes, lines and bucket counts are checked: G2P_E_ARG otherwise).  *out is
+ *                          double-buffered per context like the *_host results; res->n_loaded / n_filtered count the chunk.
+ * load and emit calls of chunks on different contexts may run concurrently from different host threads.
+ * G2P_FILTER_PARTS=k (tests) forces at least k partitions. */
+typedef struct g2p_filter_job g2p_filter_job;
+typedef struct g2p_filter_job_stats {
+    double load_ms, decide_ms, emit_ms;   /* CUDA-event time summed over the calls of each pass */
+    uint64_t h2d_bytes, d2h_bytes;        /* bytes copied over PCIe by the job's calls */
+} g2p_filter_job_stats;
+int g2p_filter_job_create(g2p_ctx* const* ctxs, int nctx, const g2p_filter_params* params, g2p_filter_job** out);
+int g2p_filter_job_load(g2p_filter_job* job, uint64_t chunk, const char* text, size_t n);
+int g2p_filter_job_decide(g2p_filter_job* job, g2p_filter_result* res);
+int g2p_filter_job_emit(g2p_filter_job* job, uint64_t chunk, const char* text, size_t n, const char** out, g2p_filter_result* res);
+int g2p_filter_job_get_stats(const g2p_filter_job* job, g2p_filter_job_stats* stats);
+void g2p_filter_job_destroy(g2p_filter_job* job);
+
 /* Formats the stderr line the reference prints for a failed record (empty for aborts,
  * whose text comes from the C++ runtime).  `gaf` is the host copy of the input. */
 int g2p_format_error(const g2p_result* res, const char* gaf, size_t n, char* buf, size_t cap);
