@@ -927,6 +927,7 @@ int g2p_convert_host(g2p_ctx* ctx, const char* gaf, size_t n, const char** out, 
         res->device_ms += r.device_ms; res->emit_ms += r.emit_ms; res->size_ms += r.size_ms; res->index_ms += r.index_ms;
         res->fused_ms += r.fused_ms; res->n_fused += r.n_fused;
         res->n_delegated += r.n_delegated; res->n_long += r.n_long;
+        res->par_ms += r.par_ms; res->n_par += r.n_par;
     }
     res->out_bytes = S.off[last + 1];
     if (S.stop_at < nchunks) {
