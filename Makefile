@@ -41,7 +41,7 @@ $(BUILD)/gafgen: tools/gafgen.cpp
 	@mkdir -p $(BUILD)
 	$(CXX) $(CXXFLAGS) -DGAFGEN_MAIN -pthread -o $@ $<
 
-hostsim: $(BUILD)/g2p_hostsim $(BUILD)/g2p_simt $(BUILD)/g2p_simt_long $(BUILD)/g2u_hostsim $(BUILD)/g2u_simt $(BUILD)/g2u_simt_small $(BUILD)/gaf2paf_stub $(BUILD)/g2p_filter_simt $(BUILD)/g2p_filter_job_simt $(BUILD)/g2p_floatparse
+hostsim: $(BUILD)/g2p_hostsim $(BUILD)/g2p_simt $(BUILD)/g2p_simt_long $(BUILD)/g2u_hostsim $(BUILD)/g2u_simt $(BUILD)/g2u_simt_small $(BUILD)/gaf2paf_stub $(BUILD)/gaf2unstable_stub $(BUILD)/g2p_filter_simt $(BUILD)/g2p_filter_job_simt $(BUILD)/g2p_floatparse
 $(BUILD)/g2p_filter_simt: tests/hostsim/g2p_filter_simt.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -Itests/hostsim -o $@ $<
@@ -51,10 +51,13 @@ $(BUILD)/g2p_filter_job_simt: tests/hostsim/g2p_filter_job_simt.cpp tests/hostsi
 $(BUILD)/g2p_floatparse: tests/hostsim/g2p_floatparse.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -Itests/hostsim -o $@ $<
-# the gaf2paf executable's host logic linked against a CPU stub of the C-ABI (test infrastructure)
+# the gaf2paf and gaf2unstable executables' host logic linked against CPU stubs of the C-ABI (test infrastructure)
 $(BUILD)/gaf2paf_stub: $(CSRC)/gaf2paf_main.cpp $(CSRC)/cli_pipeline.hpp tests/hostsim/g2p_stub_capi.cpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) $(CXXFLAGS) -ffp-contract=off -pthread -o $@ $(CSRC)/gaf2paf_main.cpp tests/hostsim/g2p_stub_capi.cpp
+$(BUILD)/gaf2unstable_stub: $(CSRC)/gaf2unstable_main.cpp $(CSRC)/cli_pipeline.hpp tests/hostsim/g2u_stub_capi.cpp $(HDRS)
+	@mkdir -p $(BUILD)
+	$(CXX) $(CXXFLAGS) -ffp-contract=off -pthread -o $@ $(CSRC)/gaf2unstable_main.cpp tests/hostsim/g2u_stub_capi.cpp
 $(BUILD)/g2u_hostsim: tests/hostsim/g2u_hostsim.cpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) $(CXXFLAGS) -ffp-contract=off -o $@ $<

@@ -37,7 +37,7 @@ REC_ABORT = 16
 EXPORTED_SYMBOLS = (
     "g2p_create", "g2p_destroy", "g2p_last_error", "g2p_host_alloc", "g2p_host_free", "g2p_load_lengths",
     "g2p_table_entries", "g2p_copy_to_device", "g2p_copy_to_host", "g2p_convert_device", "g2p_convert_host", "g2p_index_lines", "g2p_format_error",
-    "g2p_load_rgfa", "g2p_rgfa_node_lengths", "g2p_unstable_device", "g2p_unstable_host", "g2p_unstable_warnings", "g2p_format_unstable_warning",
+    "g2p_load_rgfa", "g2p_share_rgfa", "g2p_rgfa_node_lengths", "g2p_unstable_device", "g2p_unstable_host", "g2p_unstable_warnings", "g2p_format_unstable_warning",
     "g2p_unstable_convert_device", "g2p_unstable_convert_host", "g2p_unstable_convert_warnings",
     "g2p_filter_device", "g2p_filter_host",
     "g2p_filter_job_create", "g2p_filter_job_load", "g2p_filter_job_decide", "g2p_filter_job_emit", "g2p_filter_job_get_stats",
@@ -135,6 +135,8 @@ def _load():
     lib.g2p_format_error.restype = ctypes.c_int
     lib.g2p_load_rgfa.argtypes = [vp, vp, sz, ctypes.POINTER(ctypes.c_int), vp, sz]
     lib.g2p_load_rgfa.restype = ctypes.c_int
+    lib.g2p_share_rgfa.argtypes = [vp, vp]
+    lib.g2p_share_rgfa.restype = ctypes.c_int
     lib.g2p_rgfa_node_lengths.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(sz)]
     lib.g2p_rgfa_node_lengths.restype = ctypes.c_int
     lib.g2p_unstable_device.argtypes = [vp, vp, sz, ctypes.POINTER(vp), ctypes.POINTER(Result), vp]
@@ -268,6 +270,11 @@ class Converter:
             return False, code.value, msg.value.decode("latin-1")
         self._check(rc)
         return True, 0, ""
+
+    def share_rgfa(self, src):
+        """Take the rGFA tables ``src`` (another :class:`Converter`) loaded with :meth:`load_rgfa`, without reading the
+        rGFA again (g2p_share_rgfa).  Raises :class:`G2PError` when ``src`` has none."""
+        self._check(lib.g2p_share_rgfa(self._h, src._h))
 
     def node_lengths(self):
         """Contents of the -o file of gaf2unstable."""

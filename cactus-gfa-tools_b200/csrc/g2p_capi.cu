@@ -25,7 +25,7 @@
 #include "../../include/g2p.h"
 #include "g2p_kernels.cuh"
 #include "g2p_table.hpp"
-#include "g2u_rgfa.hpp"
+#include "g2u_tables.hpp"
 #include "g2p_errfmt.hpp"
 #include "g2p_filter_job.hpp"
 #include <memory>
@@ -137,8 +137,7 @@ struct g2p_ctx {
     bool warn_pending = false;
     UnstableView uview{};
     bool have_rgfa = false;
-    RgfaTables* rgfa = nullptr;
-    std::string node_lengths;
+    std::shared_ptr<const RgfaHost> rgfa;   // host copy of the tables, shared by every context they were given to
     std::vector<g2p_warn> warns;
     size_t host_chunk = kHostChunk;
     bool host_chunk_fixed = false;   // G2P_HOST_CHUNK_MB given: no adaptation to the record length
@@ -293,7 +292,6 @@ void g2p_destroy(g2p_ctx* ctx) {
     ctx->d_slots.release();
     ctx->d_arena.release();
     for (DevBuf* b : {&ctx->u_slots, &ctx->u_arena, &ctx->u_begin, &ctx->u_nodes, &ctx->u_names, &ctx->u_refoff, &ctx->u_refnames, &ctx->n_slots, &ctx->n_arena}) b->release();
-    delete ctx->rgfa;
     for (auto& w : ctx->w) w.release();
     for (auto& b : ctx->h_outs) b.release();
     delete ctx;
@@ -944,15 +942,51 @@ int g2p_convert_host(g2p_ctx* ctx, const char* gaf, size_t n, const char** out, 
 // ---------------------------------------------------------------------------------------
 // gaf2unstable
 // ---------------------------------------------------------------------------------------
+// Uploads the tables of H into ctx's buffers: the one upload path of g2p_load_rgfa and g2p_share_rgfa.
+static int upload_rgfa(g2p_ctx* ctx, const std::shared_ptr<const RgfaHost>& H) {
+    G2P_CUDA(cudaSetDevice(ctx->device));
+    ctx->rgfa = H;
+    ctx->have_rgfa = false;
+    G2P_CUDA(cudaDeviceSynchronize());
+    auto up = [&](DevBuf& b, const void* src, size_t bytes) -> cudaError_t {
+        cudaError_t e = b.ensure(bytes ? bytes : 16);
+        if (e != cudaSuccess) return e;
+        return bytes ? cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) : cudaSuccess;
+    };
+    G2P_CUDA(up(ctx->u_slots, H->contigs.slots.data(), H->contigs.slots.size() * sizeof(LenSlot)));
+    G2P_CUDA(up(ctx->u_arena, H->contigs.arena.data(), H->contigs.arena.size()));
+    G2P_CUDA(up(ctx->u_begin, H->begin.data(), H->begin.size() * sizeof(u32)));
+    G2P_CUDA(up(ctx->u_nodes, H->nodes.data(), H->nodes.size() * sizeof(UNode)));
+    G2P_CUDA(up(ctx->u_names, H->names.data(), H->names.size()));
+    G2P_CUDA(up(ctx->u_refoff, H->refoff.data(), H->refoff.size() * sizeof(u32)));
+    G2P_CUDA(up(ctx->u_refnames, H->refnames.data(), H->refnames.size()));
+    ctx->uview.contigs.slots = static_cast<const LenSlot*>(ctx->u_slots.p);
+    ctx->uview.contigs.arena = static_cast<const u8*>(ctx->u_arena.p);
+    ctx->uview.contigs.nslots = (u32)H->contigs.slots.size();
+    ctx->uview.contig_begin = static_cast<const u32*>(ctx->u_begin.p);
+    ctx->uview.nodes = static_cast<const UNode*>(ctx->u_nodes.p);
+    ctx->uview.node_names = static_cast<const u8*>(ctx->u_names.p);
+    ctx->uview.ref_off = static_cast<const u32*>(ctx->u_refoff.p);
+    ctx->uview.ref_names = static_cast<const u8*>(ctx->u_refnames.p);
+    // the node-lengths table of the fused gaf2unstable | gaf2paf path
+    G2P_CUDA(up(ctx->n_slots, H->node_table.slots.data(), H->node_table.slots.size() * sizeof(LenSlot)));
+    G2P_CUDA(up(ctx->n_arena, H->node_table.arena.data(), H->node_table.arena.size()));
+    ctx->node_table.slots = static_cast<const LenSlot*>(ctx->n_slots.p);
+    ctx->node_table.arena = static_cast<const u8*>(ctx->n_arena.p);
+    ctx->node_table.nslots = (u32)H->node_table.slots.size();
+    ctx->have_rgfa = true;
+    return G2P_OK;
+}
+
 int g2p_load_rgfa(g2p_ctx* ctx, const char* rgfa, size_t n, int* ref_exit_code, char* msg, size_t msg_cap) {
     if (!ctx || (!rgfa && n)) return G2P_E_ARG;
     if (ref_exit_code) *ref_exit_code = 0;
     if (msg && msg_cap) msg[0] = 0;
     G2P_CUDA(cudaSetDevice(ctx->device));
-    delete ctx->rgfa;
-    ctx->rgfa = new RgfaTables();
-    RgfaTables& T = *ctx->rgfa;
-    build_rgfa_tables(rgfa, n, T);
+    auto H = std::make_shared<RgfaHost>();
+    ctx->rgfa = H;
+    const RgfaTables& T = H->T;
+    build_rgfa_tables(rgfa, n, H->T);
     if (T.exit_code) {
         if (ref_exit_code) *ref_exit_code = T.exit_code;
         if (msg && msg_cap) std::snprintf(msg, msg_cap, "%s", T.exit_code == 1 ? T.error.c_str() : "");
@@ -960,84 +994,21 @@ int g2p_load_rgfa(g2p_ctx* ctx, const char* rgfa, size_t n, int* ref_exit_code, 
         ctx->have_rgfa = false;
         return G2P_E_TABLE;
     }
-    // flatten: contig hash -> index, nodes per contig sorted by SO, names, node -> reference contig
-    HostLenTable ct;
-    ct.reserve_for(T.mapping.size());
-    std::vector<u32> begin;
-    std::vector<UNode> nodes;
-    std::vector<u8> names;
-    ctx->node_lengths.clear();
-    u32 ci = 0;
-    for (const auto& cs : T.mapping) {
-        ct.put(reinterpret_cast<const u8*>(cs.first.data()), (u32)cs.first.size(), (i64)ci++);
-        begin.push_back((u32)nodes.size());
-        i64 cum = 0;
-        for (const RgfaNode& nd : cs.second) {
-            UNode u;
-            u.offset = nd.offset; u.cum = cum; u.length = (u32)nd.length;
-            u.name_off = (u32)names.size(); u.name_len = (u32)nd.name.size();
-            names.insert(names.end(), nd.name.begin(), nd.name.end());
-            int64_t id;
-            u.ref = -1;
-            if (rgfa_detail::node_id_of(nd.name, id)) {
-                auto it = T.node_to_contig.find(id);
-                if (it != T.node_to_contig.end()) u.ref = (i32)it->second;
-            }
-            cum += nd.length;
-            nodes.push_back(u);
-            ctx->node_lengths += nd.name;
-            ctx->node_lengths += '\t';
-            ctx->node_lengths += std::to_string(nd.length);
-            ctx->node_lengths += '\n';
-        }
-    }
-    begin.push_back((u32)nodes.size());
-    if (ct.arena.empty()) ct.arena.push_back(0);
-    std::vector<u32> refoff{0};
-    std::vector<u8> refnames;
-    for (const std::string& c : T.ref_contigs) { refnames.insert(refnames.end(), c.begin(), c.end()); refoff.push_back((u32)refnames.size()); }
-    if (names.empty()) names.push_back(0);
-    if (refnames.empty()) refnames.push_back(0);
-    if (nodes.empty()) nodes.push_back(UNode{0, 0, 0, 0, 0, -1});
-    G2P_CUDA(cudaDeviceSynchronize());
-    auto up = [&](DevBuf& b, const void* src, size_t bytes) -> cudaError_t {
-        cudaError_t e = b.ensure(bytes ? bytes : 16);
-        if (e != cudaSuccess) return e;
-        return bytes ? cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) : cudaSuccess;
-    };
-    G2P_CUDA(up(ctx->u_slots, ct.slots.data(), ct.slots.size() * sizeof(LenSlot)));
-    G2P_CUDA(up(ctx->u_arena, ct.arena.data(), ct.arena.size()));
-    G2P_CUDA(up(ctx->u_begin, begin.data(), begin.size() * sizeof(u32)));
-    G2P_CUDA(up(ctx->u_nodes, nodes.data(), nodes.size() * sizeof(UNode)));
-    G2P_CUDA(up(ctx->u_names, names.data(), names.size()));
-    G2P_CUDA(up(ctx->u_refoff, refoff.data(), refoff.size() * sizeof(u32)));
-    G2P_CUDA(up(ctx->u_refnames, refnames.data(), refnames.size()));
-    ctx->uview.contigs.slots = static_cast<const LenSlot*>(ctx->u_slots.p);
-    ctx->uview.contigs.arena = static_cast<const u8*>(ctx->u_arena.p);
-    ctx->uview.contigs.nslots = (u32)ct.slots.size();
-    ctx->uview.contig_begin = static_cast<const u32*>(ctx->u_begin.p);
-    ctx->uview.nodes = static_cast<const UNode*>(ctx->u_nodes.p);
-    ctx->uview.node_names = static_cast<const u8*>(ctx->u_names.p);
-    ctx->uview.ref_off = static_cast<const u32*>(ctx->u_refoff.p);
-    ctx->uview.ref_names = static_cast<const u8*>(ctx->u_refnames.p);
-    {   // the node-lengths table of the fused gaf2unstable | gaf2paf path: exactly what `gaf2paf -l <the -o file>` would load
-        HostLenTable nt;
-        if (build_len_table(ctx->node_lengths.data(), ctx->node_lengths.size(), nt) != ST_OK) { ctx->set_err("node lengths table"); return G2P_E_TABLE; }
-        G2P_CUDA(up(ctx->n_slots, nt.slots.data(), nt.slots.size() * sizeof(LenSlot)));
-        G2P_CUDA(up(ctx->n_arena, nt.arena.data(), nt.arena.size()));
-        ctx->node_table.slots = static_cast<const LenSlot*>(ctx->n_slots.p);
-        ctx->node_table.arena = static_cast<const u8*>(ctx->n_arena.p);
-        ctx->node_table.nslots = (u32)nt.slots.size();
-    }
-    ctx->have_rgfa = true;
-    return G2P_OK;
+    if (!flatten_rgfa(*H)) { ctx->set_err("node lengths table"); ctx->have_rgfa = false; return G2P_E_TABLE; }
+    return upload_rgfa(ctx, H);
+}
+
+int g2p_share_rgfa(g2p_ctx* dst, const g2p_ctx* src) {
+    if (!dst || !src || dst == src) return G2P_E_ARG;
+    if (!src->have_rgfa) return G2P_E_NOTABLE;
+    return upload_rgfa(dst, src->rgfa);
 }
 
 int g2p_rgfa_node_lengths(g2p_ctx* ctx, const char** tsv, size_t* n) {
     if (!ctx || !tsv || !n) return G2P_E_ARG;
     if (!ctx->have_rgfa) return G2P_E_NOTABLE;
-    *tsv = ctx->node_lengths.data();
-    *n = ctx->node_lengths.size();
+    *tsv = ctx->rgfa->node_lengths.data();
+    *n = ctx->rgfa->node_lengths.size();
     return G2P_OK;
 }
 
@@ -1250,37 +1221,11 @@ int g2p_unstable_warnings(g2p_ctx* ctx, const g2p_warn** warns, size_t* n) {
     return G2P_OK;
 }
 
-// "[gaf2unstable] warning: Target path spans multiple reference contigs a, b, \nthe (unstable) record is\n<line>\n"
-// (gaf2unstable_main.cpp:165-171): contig names in ascending contig-id order; the record printed
-// there does not carry an rc tag of its own making, which is what the output line holds as well.
 int g2p_format_unstable_warning(g2p_ctx* ctx, const char* line, size_t len, char* buf, size_t cap) {
     if (!ctx || !line || !buf || cap == 0 || !ctx->rgfa) return G2P_E_ARG;
     buf[0] = 0;
-    const RgfaTables& T = *ctx->rgfa;
-    // column 6 = the path
-    size_t a = 0;
-    for (int c = 0; c < 5 && a < len; ++c) { const void* t = std::memchr(line + a, '\t', len - a); if (!t) return G2P_E_ARG; a = static_cast<const char*>(t) - line + 1; }
-    const void* te = std::memchr(line + a, '\t', len - a);
-    const size_t b = te ? static_cast<const char*>(te) - line : len;
-    std::set<int64_t> ids;
-    size_t p = a;
-    while (p < b) {
-        size_t q = p + 1;
-        while (q < b && line[q] != '>' && line[q] != '<') ++q;
-        int64_t id;
-        if (rgfa_detail::node_id_of(std::string(line + p + 1, q - p - 1), id)) {
-            auto it = T.node_to_contig.find(id);
-            if (it != T.node_to_contig.end()) ids.insert(it->second);
-        }
-        p = q;
-    }
-    std::string m = "[gaf2unstable] warning: Target path spans multiple reference contigs ";
-    for (int64_t id : ids) { m += T.ref_contigs[(size_t)id]; m += ", "; }
-    m += "\nthe (unstable) record is\n";
-    size_t ll = len;
-    while (ll > 0 && line[ll - 1] == '\n') --ll;
-    m.append(line, ll);
-    m += "\n";
+    std::string m;
+    if (!format_unstable_warning(ctx->rgfa->T, line, len, m)) return G2P_E_ARG;
     std::snprintf(buf, cap, "%s", m.c_str());
     return G2P_OK;
 }

@@ -1,24 +1,35 @@
 // gaf2unstable — drop-in command line for the reference tool of the same name
 // (reference gaf2unstable_main.cpp:177-301): same options (and option quirks), same stdout
-// bytes, same stderr messages and exit codes; the per-record rewrite runs on a B200 through
-// the C-ABI of libg2p.so (include/g2p.h), the rGFA tables are built once on the host.
+// bytes, same stderr messages and exit codes; the per-record rewrite runs on B200 GPUs through
+// the C-ABI of libg2p.so (include/g2p.h).
 //
 //   gaf2unstable [options] <gaf>
 //     -g, --rgfa FILE   (uncompressed) minigraph rGFA
 //     -o FILE           write "node<TAB>length" for every rGFA node (input of gaf2paf -l)
 //
-// Environment: G2P_DEVICE=K (device ordinal), G2P_CHUNK_MB=M (bytes of GAF per GPU call; default 16 for short records, up to 512 for long ones),
-// G2P_IO_THREADS=T.  Host side: the reader -> converter -> writer pipeline of cli_pipeline.hpp.
+// Environment (argv stays identical to the reference):
+//   G2P_GPUS=N        shard the input over the first N GPUs of the box by newline-aligned
+//                     byte ranges; outputs and warnings are printed in input order (default 1)
+//   G2P_DEVICE=K      first device ordinal (default 0)
+//   G2P_CHUNK_MB=M    bytes of GAF per GPU call (default: 16 for short records, up to 512 for long ones)
+//   G2P_IO_THREADS=T  threads of the parallel pread / pwrite of regular files
+//   G2P_STATS=1       timing summary on stderr
+//
+// The rGFA tables are built once on the host (g2p_load_rgfa on the first GPU's context, while the
+// other contexts are created) and copied to every other GPU (g2p_share_rgfa).  The host side is the
+// reader -> per-GPU converter -> writer pipeline of cli_pipeline.hpp.
 #include <fcntl.h>
 #include <getopt.h>
 #include <signal.h>
 #include <unistd.h>
 
 #include <cerrno>
+#include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "cli_pipeline.hpp"
@@ -99,21 +110,45 @@ int main(int argc, char** argv) {
         close(fd);
     }
 
-    g2p_ctx* ctx = nullptr;
-    if (g2p_create((int)cli::env_long("G2P_DEVICE", 0), &ctx) != G2P_OK) {
+    const int ngpu = (int)std::max(1L, cli::env_long("G2P_GPUS", 1));
+    const int dev0 = (int)cli::env_long("G2P_DEVICE", 0);
+    const bool stats = cli::env_long("G2P_STATS", 0) != 0;
+    using clk = std::chrono::steady_clock;
+    auto secs = [](clk::time_point t) { return std::chrono::duration<double>(clk::now() - t).count(); };
+
+    // one context per GPU, created concurrently (CUDA context creation is the bulk of the start-up time); the first one
+    // builds the rGFA tables meanwhile
+    std::vector<g2p_ctx*> ctx(ngpu, nullptr);
+    std::vector<int> crc(ngpu, G2P_OK);
+    std::vector<std::thread> th;
+    for (int g = 1; g < ngpu; ++g) th.emplace_back([&, g] { crc[g] = g2p_create(dev0 + g, &ctx[g]); });
+    crc[0] = g2p_create(dev0, &ctx[0]);
+    int ref_rc = 0, rc = G2P_OK;
+    std::vector<char> msg(1 << 16);
+    double load_s = 0;
+    if (crc[0] == G2P_OK) {
+        const auto t = clk::now();
+        rc = g2p_load_rgfa(ctx[0], rgfa.data(), rgfa.size(), &ref_rc, msg.data(), msg.size());
+        load_s = secs(t);
+    }
+    for (auto& t : th) t.join();
+    th.clear();
+    if (crc[0] != G2P_OK) {
         fprintf(stderr, "[gaf2unstable] error: no usable CUDA device (this build has no CPU path)\n");
         return 1;
     }
-    int ref_rc = 0;
-    std::vector<char> msg(1 << 16);
-    int rc = g2p_load_rgfa(ctx, rgfa.data(), rgfa.size(), &ref_rc, msg.data(), msg.size());
     if (rc == G2P_E_TABLE) {
         fputs(msg.data(), stderr);
         if (ref_rc == 1) return 1;
         abort();
     }
-    if (rc != G2P_OK) { fprintf(stderr, "[gaf2unstable] error: %s\n", g2p_last_error(ctx)); return 1; }
+    if (rc != G2P_OK) { fprintf(stderr, "[gaf2unstable] error: %s\n", g2p_last_error(ctx[0])); return 1; }
     std::string().swap(rgfa);
+    for (int g = 1; g < ngpu; ++g)
+        if (crc[g] != G2P_OK) {
+            fprintf(stderr, "[gaf2unstable] error: no usable CUDA device %d (this build has no CPU path)\n", dev0 + g);
+            return 1;
+        }
 
     if (!node_lengths_path.empty()) {
         FILE* o = fopen(node_lengths_path.c_str(), "wb");
@@ -123,10 +158,19 @@ int main(int argc, char** argv) {
         }
         const char* tsv = nullptr;
         size_t n = 0;
-        g2p_rgfa_node_lengths(ctx, &tsv, &n);
+        g2p_rgfa_node_lengths(ctx[0], &tsv, &n);
         fwrite(tsv, 1, n, o);
         fclose(o);
     }
+
+    // the tables of the first context go to the others: no second pass over the rGFA
+    const auto t_share = clk::now();
+    std::vector<int> src(ngpu, G2P_OK);
+    for (int g = 1; g < ngpu; ++g) th.emplace_back([&, g] { src[g] = g2p_share_rgfa(ctx[g], ctx[0]); });
+    for (auto& t : th) t.join();
+    const double share_s = secs(t_share);
+    for (int g = 1; g < ngpu; ++g)
+        if (src[g] != G2P_OK) { fprintf(stderr, "[gaf2unstable] error: %s\n", g2p_last_error(ctx[g])); return 1; }
 
     size_t chunk = (size_t)std::max(1L, cli::env_long("G2P_CHUNK_MB", 16)) << 20;
     if (cli::env_long("G2P_CHUNK_BYTES", 0) > 0) chunk = (size_t)cli::env_long("G2P_CHUNK_BYTES", 0);   // tests: tiny chunks
@@ -134,7 +178,7 @@ int main(int argc, char** argv) {
     P.tool = "gaf2unstable";
     P.chunk_bytes = chunk;
     P.chunk_auto = !getenv("G2P_CHUNK_MB") && !getenv("G2P_CHUNK_BYTES");
-    P.ctx.push_back(ctx);
+    P.ctx = ctx;
     P.convert = [](g2p_ctx* cx, cli::Chunk& c) {
         int r = g2p_unstable_host(cx, c.buf, c.n, &c.out, &c.res);
         if (r != G2P_OK) return r;
@@ -156,7 +200,13 @@ int main(int argc, char** argv) {
         fflush(stderr);
         abort();   // reference: assert / uncaught exception -> SIGABRT
     };
+    const auto t0 = clk::now();
+    if (stats) fprintf(stderr, "[gaf2unstable] stats: contexts ready\n");
     const int prc = P.run({in_gaf_path});
-    g2p_destroy(ctx);
+    if (stats)
+        fprintf(stderr, "[gaf2unstable] stats: records=%llu in=%llu B out=%llu B device=%.3f ms wall=%.3f s gpus=%d rgfa=%.3f s share=%.3f s\n",
+                (unsigned long long)P.tot_rec, (unsigned long long)P.tot_in, (unsigned long long)P.tot_out, P.device_ms, secs(t0), ngpu, load_s,
+                share_s);
+    for (g2p_ctx* c : P.ctx) g2p_destroy(c);
     return prc;
 }

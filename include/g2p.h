@@ -124,8 +124,17 @@ int g2p_index_lines(g2p_ctx* ctx, const void* d_text, size_t n, const uint32_t**
  * (exit 1 cases) in msg. */
 int g2p_load_rgfa(g2p_ctx* ctx, const char* rgfa, size_t n, int* ref_exit_code, char* msg, size_t msg_cap);
 
+/* Gives dst the tables src loaded with g2p_load_rgfa, without reading the rGFA again: the host copy
+ * of the flat arrays that call built is kept (and shared between the contexts) and uploaded to dst's
+ * device; g2p_rgfa_node_lengths and the warnings of dst then come from the same tables.  Several
+ * calls with one src and different dst may run concurrently from different host threads, while
+ * nothing else uses src.  G2P_E_ARG for a null context or dst == src, G2P_E_NOTABLE when src has no
+ * tables, G2P_E_CUDA when a copy fails. */
+int g2p_share_rgfa(g2p_ctx* dst, const g2p_ctx* src);
+
 /* Contents of the -o node-lengths file (gaf2unstable_main.cpp:274-285), rows in the
- * reference's order.  Library-owned, valid until the next g2p_load_rgfa / g2p_destroy. */
+ * reference's order.  Library-owned, valid until the next g2p_load_rgfa / g2p_share_rgfa /
+ * g2p_destroy on this context. */
 int g2p_rgfa_node_lengths(g2p_ctx* ctx, const char** tsv, size_t* n);
 
 /* Replaces the record loop of gaf2unstable main() (gaf2unstable_main.cpp:288-297) with
