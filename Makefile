@@ -66,7 +66,7 @@ $(BUILD)/g2u_simt: tests/hostsim/g2u_hostsim.cpp tests/hostsim/cuda_shim.hpp $(H
 	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -DG2U_SIMT -Itests/hostsim -o $@ $<
 $(BUILD)/g2u_simt_small: tests/hostsim/g2u_hostsim.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
 	@mkdir -p $(BUILD)
-	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -DG2U_SIMT -DG2U_IN_CAP=4096u -DG2U_OUT_CAP=6144u -Itests/hostsim -o $@ $<
+	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -DG2U_SIMT -DG2U_SIMT_STAGED_ONLY=1 -DG2U_IN_CAP=4096u -DG2U_OUT_CAP=6144u -Itests/hostsim -o $@ $<
 $(BUILD)/g2p_simt_long: tests/hostsim/g2p_simt.cpp tests/hostsim/cuda_shim.hpp $(HDRS)
 	@mkdir -p $(BUILD)
 	$(CXX) -O1 -g -std=c++17 -ffp-contract=off -Wall -Wno-unused-function -Wno-unknown-pragmas -DG2P_S_LIMIT=0 -Itests/hostsim -o $@ $<

@@ -133,7 +133,8 @@ struct g2p_ctx {
     DevBuf n_slots, n_arena;              // node name -> length table of the rGFA (what gaf2unstable -o writes, loaded like gaf2paf -l)
     LenTableView node_table{nullptr, nullptr, 0};
     std::string warn_text;                // stderr text of the gaf2unstable stage of the last g2p_unstable_convert_* call
-    const u8* warn_mid = nullptr;         // (built on demand from the intermediate GAF, which stays in the worker's d_mid buffer)
+    const u8* warn_mid = nullptr;         // (built on demand from the intermediate GAF, which stays in the worker's d_mid buffer,
+    std::vector<g2p_warn> mid_warns;      // and from that call's own copy of its warning list: g2p_unstable_* replaces `warns`)
     bool warn_pending = false;
     UnstableView uview{};
     bool have_rgfa = false;
@@ -1134,12 +1135,22 @@ static int run_unstable_convert(g2p_ctx* ctx, Worker& w, const u8* d_gaf, size_t
     g2p_result r1;
     u8* d_mid = nullptr;
     ctx->warn_text.clear();
+    ctx->mid_warns.clear();
+    ctx->warn_pending = false;
     int rc = run_unstable(ctx, w, d_gaf, n, st, &r1, &d_mid);
     if (rc) return rc;
     (void)d_mid;
+    // stage 2 indexes its input with 32-bit offsets, like every gaf2paf entry point; stage 1 writes one node name per node
+    // an interval covers, so a small input can expand past that
+    if (r1.out_bytes >= 0xFFFFFFF0ULL) {
+        ctx->set_err("the intermediate GAF of gaf2unstable is " + std::to_string(r1.out_bytes) +
+                     " bytes; the gaf2paf stage takes less than 4 GiB: split the input");
+        return G2P_E_TOOBIG;
+    }
     std::swap(w.d_out, w.d_mid);   // the intermediate GAF stays in d_mid (until the next call); the converter writes d_out
     ctx->warn_mid = static_cast<const u8*>(w.d_mid.p);
-    ctx->warn_pending = !ctx->warns.empty();
+    ctx->mid_warns = ctx->warns;
+    ctx->warn_pending = !ctx->mid_warns.empty();
     const LenTableView saved = ctx->table;
     const bool saved_have = ctx->have_table;
     ctx->table = ctx->node_table;
@@ -1201,7 +1212,7 @@ int g2p_unstable_convert_warnings(g2p_ctx* ctx, const char** text, size_t* n) {
         // the stage-1 warnings (gaf2unstable_main.cpp:165-171) quote the record it wrote: fetch those lines from the
         // intermediate GAF -- here, not inside the conversion call
         G2P_CUDA(cudaSetDevice(ctx->device));
-        for (const g2p_warn& wn : ctx->warns) {
+        for (const g2p_warn& wn : ctx->mid_warns) {
             std::vector<char> line(wn.out_len + 1), msg(wn.out_len + 4096);
             G2P_CUDA(cudaMemcpy(line.data(), ctx->warn_mid + wn.out_off, wn.out_len, cudaMemcpyDeviceToHost));
             g2p_format_unstable_warning(ctx, line.data(), wn.out_len, msg.data(), msg.size());

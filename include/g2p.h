@@ -161,10 +161,14 @@ int g2p_format_unstable_warning(g2p_ctx* ctx, const char* out_line, size_t len, 
  * memory, stage 2 (gaf2paf_main.cpp:134-264) converts it from there with the node lengths of the same rGFA as its
  * lengths table -- the intermediate text makes no device->host->device round trip.  Needs g2p_load_rgfa; the -l table
  * of g2p_load_lengths is not touched.  Output: the PAF bytes of the pipeline; res->stage tells which stage stopped at
- * a record (stage 1: the reference's gaf2unstable aborts; the records before it are converted). */
+ * a record (stage 1: the reference's gaf2unstable aborts; the records before it are converted).
+ * Stage 1 writes one node name per node that a stable interval covers, so its output can be much larger than its input.
+ * When that intermediate GAF (or, when stage 1 stops at a record, the part before it) is 4 GiB or more, the call returns
+ * G2P_E_TOOBIG before stage 2 runs: split the input. */
 int g2p_unstable_convert_device(g2p_ctx* ctx, const void* d_gaf, size_t n, void** d_out, g2p_result* res, void* stream);
 int g2p_unstable_convert_host(g2p_ctx* ctx, const char* gaf, size_t n, const char** out, g2p_result* res);
-/* stderr text of the gaf2unstable stage of the last g2p_unstable_convert_* call (its multi-contig warnings). */
+/* stderr text of the gaf2unstable stage of the last g2p_unstable_convert_* call (its multi-contig warnings).  Calls of
+ * g2p_unstable_device / _host in between do not change it. */
 int g2p_unstable_convert_warnings(g2p_ctx* ctx, const char** text, size_t* n);
 
 /* ---- gaffilter (SURVEY.md §8f N1): the query-overlap filter on GAF or PAF text that is already on the device ----------

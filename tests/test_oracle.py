@@ -2,6 +2,7 @@
 against the committed golden vectors and, where the reference build is present,
 against the reference binary on seeded synthetic inputs."""
 import os
+import subprocess
 import tempfile
 
 import pytest
@@ -97,21 +98,37 @@ def test_unterminated_last_line_and_two_files():
 
 # ---- gaf2unstable (config 2) ---------------------------------------------------------------
 G2U_HOSTSIM = os.path.join(H.BUILD, "g2u_hostsim")
-G2U_SIMT = os.path.join(H.BUILD, "g2u_simt")   # k_unstable_staged<> itself under the SIMT emulator
+G2U_SIMT = os.path.join(H.BUILD, "g2u_simt")   # k_unstable<> (G2U_SIMT_STAGED=1: k_unstable_staged<>) under the SIMT emulator
 G2U_PORT = os.path.join(H.ORACLE_BIN, "gaf2unstable_oracle")
+# the kernels under the emulator: k_unstable, the library's default, over a grid of 3 CTAs (several stride turns), also
+# with the CTAs in reverse order (the warning list fills in another order); k_unstable_staged; the staged kernel with
+# tiny staging buffers (_small), so that some CTAs read / write global memory directly
+G2U_SIMT_RUNS = {
+    "list": (G2U_SIMT, {}),
+    "list-reverse": (G2U_SIMT, {"G2P_SIMT_REVERSE": "1"}),
+    "staged": (G2U_SIMT, {"G2U_SIMT_STAGED": "1"}),
+    "staged-small": (G2U_SIMT + "_small", {}),
+}
 
 
-@pytest.mark.parametrize("binary", [G2U_HOSTSIM, G2U_SIMT, G2U_PORT])
-def test_gaf2unstable_host_code_matches_golden(binary):
+def run_g2u(binary, args, stdin, env=None):
+    """-> (exit code, stdout, stderr text) of a gaf2unstable stand-in with `env` added to the environment."""
+    p = subprocess.run([binary] + args, input=stdin, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=dict(os.environ, **(env or {})))
+    return (p.returncode if p.returncode >= 0 else 128 - p.returncode), p.stdout, p.stderr.decode("latin-1")
+
+
+@pytest.mark.parametrize("run", ["hostsim", "port"] + sorted(G2U_SIMT_RUNS))
+def test_gaf2unstable_host_code_matches_golden(run):
     """the device code on the host, and the independent oracle restatement, against the golden vectors"""
+    binary, env = {"hostsim": (G2U_HOSTSIM, {}), "port": (G2U_PORT, {})}.get(run) or G2U_SIMT_RUNS[run]
     d = H.golden("gaf2unstable_kat.json")
     with tempfile.TemporaryDirectory() as td:
         gp, lp = os.path.join(td, "g.gfa"), os.path.join(td, "nl.tsv")
         open(gp, "w").write(d["rgfa"])
         for v in d["vectors"]:
-            rc, out, err = H.run_tool(binary, ["-g", gp, "-"], (v["in"] + "\n").encode())
+            rc, out, err = run_g2u(binary, ["-g", gp, "-"], (v["in"] + "\n").encode(), env)
             assert rc == v["rc"] and out.decode() == v["out"], v["in"]
-        rc, out, err = H.run_tool(binary, ["-g", gp, "-o", lp, "-"], ("\n".join(d["stream"]["in"]) + "\n").encode())
+        rc, out, err = run_g2u(binary, ["-g", gp, "-o", lp, "-"], ("\n".join(d["stream"]["in"]) + "\n").encode(), env)
         assert rc == 0 and out.decode() == d["stream"]["out"]
         assert open(lp).read() == d["node_lengths"]
 
@@ -123,13 +140,14 @@ def test_gaf2unstable_differential(seed, aligned):
     rgfa, gaf = H.gen_rgfa_case(seed, n_records=600, aligned=aligned)
     rc, ref, err, nl = H.run_gaf2unstable_ref(gaf, rgfa, True)
     assert rc == 0
+    assert err.count("[gaf2unstable] warning") > 3
     with tempfile.TemporaryDirectory() as td:
         gp, lp = os.path.join(td, "g.gfa"), os.path.join(td, "nl.tsv")
         open(gp, "wb").write(rgfa)
-        for binary in (G2U_HOSTSIM, G2U_SIMT, G2U_SIMT + "_small"):   # _small: tiny staging buffers, so that some CTAs read / write global memory directly
-            rc, out, serr = H.run_tool(binary, ["-g", gp, "-o", lp, "-"], gaf)
-            assert rc == 0 and out == ref and open(lp, "rb").read() == nl, binary
-            assert serr.count("warning") == err.count("[gaf2unstable] warning"), binary
+        for name, (binary, env) in [("hostsim", (G2U_HOSTSIM, {}))] + sorted(G2U_SIMT_RUNS.items()):
+            rc, out, serr = run_g2u(binary, ["-g", gp, "-o", lp, "-"], gaf, env)
+            assert rc == 0 and out == ref and open(lp, "rb").read() == nl, name
+            assert serr == err, name   # the warnings verbatim and in record order
         rc, out, serr = H.run_tool(G2U_PORT, ["-g", gp, "-o", lp, "-"], gaf)   # oracle restatement: stderr verbatim too
         assert rc == 0 and out == ref and open(lp, "rb").read() == nl and serr == err
 
@@ -211,7 +229,8 @@ def test_gaf2unstable_many_tags():
         for c in cases:
             data = base[4] + b"\n" + c + b"\n" + base[5] + b"\n"
             rc, ref, err = H.run_tool(ref_bin, ["-g", gp, "-"], data)
-            for binary in (G2U_HOSTSIM, G2U_SIMT) + ((G2U_PORT,) if ref_bin != G2U_PORT else ()):
-                rc1, out1, _ = H.run_tool(binary, ["-g", gp, "-"], data)
-                assert rc1 == rc, (binary, c)
-                assert (out1 == ref) if rc == 0 else ref.startswith(out1) or out1.startswith(ref), (binary, c)
+            runs = [(G2U_HOSTSIM, {})] + list(G2U_SIMT_RUNS.values()) + ([(G2U_PORT, {})] if ref_bin != G2U_PORT else [])
+            for binary, env in runs:
+                rc1, out1, _ = run_g2u(binary, ["-g", gp, "-"], data, env)
+                assert rc1 == rc, (binary, env, c)
+                assert (out1 == ref) if rc == 0 else ref.startswith(out1) or out1.startswith(ref), (binary, env, c)
