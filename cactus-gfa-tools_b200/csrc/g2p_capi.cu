@@ -254,7 +254,7 @@ int g2p_create(int device, g2p_ctx** out) {
     if (const char* c = std::getenv("G2P_SIZE_KERNEL")) ctx->size_kernel_short = std::strcmp(c, "short") == 0;
     if (const char* c = std::getenv("G2P_LEN_SORT")) ctx->len_sort = std::atoi(c) != 0;
     if (const char* c = std::getenv("G2P_REC_CHUNKS")) ctx->rec_chunks_override = (u32)std::min(std::max(std::atoi(c), (int)kRMinChunks), (int)kRMaxChunks);
-    cudaFuncSetAttribute(k_emit_lines<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmitSmem);
+    cudaFuncSetAttribute(k_emit_lines<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmitSmemMap);
     cudaFuncSetAttribute(k_emit_lines<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmitSmem);
     cudaFuncSetAttribute(k_long<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)long_smem<true>());
     cudaFuncSetAttribute(k_long<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)long_smem<false>());
@@ -721,7 +721,7 @@ static int run_pipeline(g2p_ctx* ctx, Worker& w, const u8* d_gaf, size_t n, cuda
         if (hm->lines_total > 0xFFFFFF00ULL) { ctx->set_err("too many PAF lines in one call: split the input"); return G2P_E_TOOBIG; }
         const u32 nl = (u32)hm->lines_total;
         EmitArgs ea{d_gaf, (u64)n, d_rec, d_off, d_sdesc, d_map, d_rdesc, d_status, nl, d_o};
-        k_emit_lines<false><<<(nl + kEThreads - 1) / kEThreads, kEThreads, kEmitSmem, st>>>(ea);
+        k_emit_lines<false><<<(nl + kEThreads - 1) / kEThreads, kEThreads, kEmitSmemMap, st>>>(ea);
         ++launches;
     }
     const u32 half = desc_cap_now / 2u;

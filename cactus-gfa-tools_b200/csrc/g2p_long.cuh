@@ -585,7 +585,7 @@ __device__ __forceinline__ void long_record(const LongArgs& a, LWarpMemT<EMIT>* 
                     S.rc = head_cached ? wm->rc : rt + R.rc_a;
                     S.name = ss.src(t.name_a, t.nl);
                     S.mid = os.src(s + Ls.mid_a, Ls.mid_b - Ls.mid_a);
-                    write_line((staged ? wm->out + pad + (lincl - line) : a.out + ob + (lincl - line)) + line, S, R, Ls);
+                    write_line<false>((staged ? wm->out + pad + (lincl - line) : a.out + ob + (lincl - line)) + line, S, R, Ls);
                 }
                 if (staged) {
                     __syncwarp();

@@ -245,6 +245,39 @@ __device__ __forceinline__ u8* rput_bytes(u8* p, const u8* s, u32 n) {
     for (u32 i = n; i-- > 0;) *--p = s[i];
     return p;
 }
+// The n bytes of a run of whole CIGAR tokens ("digits letter" with at most 8 digits, which every size pass checks) at
+// src go to dst (either at any alignment), in text order or, with rev, in reverse token order with each token
+// forwards: the byte at position i of the token [s, e] goes to dst[n-1-e + i-s].  The text is read as the aligned
+// 32-bit words that hold it (never a word past it), four bytes per step; the token ends come from a rolling mask of
+// the op letters among the next 12 bytes.  So every lane runs the same flat loop whatever the direction and the token
+// structure of its text, where the nested scan-and-copy loops ran at 2-5 of 32 lanes on short-read lines.
+__device__ __forceinline__ void put_tokens(u8* dst, const u8* src, u32 n, bool rev) {
+    const uintptr_t sa = reinterpret_cast<uintptr_t>(src);
+    const u32* sp = reinterpret_cast<const u32*>(sa & ~(uintptr_t)3);
+    const u32 s8 = (u32)(sa & 3u) * 8u;
+    const u32 na = n ? ((u32)(sa & 3u) + n + 3u) >> 2 : 0u;   // aligned words that hold the text
+    auto ld = [&](u32 j) -> u32 { return j < na ? sp[j] : 0u; };
+    auto letters = [](u32 w) -> u32 { return movemask4(nondigit_bytes(w)); };
+    const u32 x0 = ld(0), x1 = ld(1), x2 = ld(2);
+    u32 x3 = ld(3);
+    u32 w0 = __funnelshift_r(x0, x1, s8), w1 = __funnelshift_r(x1, x2, s8), w2 = __funnelshift_r(x2, x3, s8);
+    u32 roll = letters(w0) | (letters(w1) << 4) | (letters(w2) << 8);   // bit t: byte 4k + t is an op letter
+    u32 s = 0;                                                          // start of the token that byte 4k is in
+    for (u32 k = 0; 4u * k < n; ++k) {
+#pragma unroll
+        for (u32 b = 0; b < 4; ++b) {
+            const u32 i = 4u * k + b;
+            const u32 below = roll & ((1u << b) - 1u);
+            const u32 ts = below ? 4u * k + 32u - (u32)__clz((int)below) : s;   // token start
+            const u32 te = i + (u32)__ffs((int)(roll >> b)) - 1u;                // its op letter
+            if (i < n) dst[rev ? n - 1u - te + i - ts : i] = (u8)(w0 >> (8u * b));
+        }
+        if (roll & 0xfu) s = 4u * k + 32u - (u32)__clz((int)(roll & 0xfu));
+        const u32 x4 = ld(k + 4u);
+        w0 = w1; w1 = w2; w2 = __funnelshift_r(x3, x4, s8); x3 = x4;
+        roll = (roll >> 4) | (letters(w2) << 8);
+    }
+}
 __device__ __forceinline__ u8* rput_tag(u8* p, u8 a, u8 b, u8 t) {   // "\tab:t:"
     p -= 6;
     p[0] = '\t'; p[1] = a; p[2] = b; p[3] = ':'; p[4] = t; p[5] = ':';
@@ -263,24 +296,28 @@ __device__ __forceinline__ LineSrc line_src(const u8* rt, const LineRec& R, cons
     S.qname = rt; S.name = rt + L.name_a; S.tp = rt + R.tp_a; S.rc = rt + R.rc_a; S.mid = rt + L.mid_a;
     return S;
 }
-// Writes the line that ends at `pend` (exclusive); returns its first byte.
+// Writes the line that ends at `pend` (exclusive); returns its first byte.  FLAT_MID: the verbatim CIGAR middle is
+// printed by put_tokens once the other fields are written; else by byte loops, a token scan nested in a per-token copy
+// for a reversed middle.  The flat loop pays on short-read lines (k_emit_lines<false>: emit 2.39 -> 2.21 ms per 10 M
+// records on a B200) and costs on the long middles of 2 kB records (k_emit_lines<true>: 3.39 -> 3.62 ms).
+template <bool FLAT_MID>
 __device__ __forceinline__ u8* write_line(u8* pend, const LineSrc& S, const LineRec& R, const LineStep& L) {
     u8* p = pend;
     *--p = '\n';
     // pieces, reversed for '<' steps (gaf2paf_main.cpp:184-211); here in reverse output order
     if (!L.rev) { *--p = L.codeE; p = rput_u32(p, L.lenE); }
     else if (L.codeS) { *--p = L.codeS; p = rput_u32(p, L.lenS); }
-    if (L.mid_b > L.mid_a) {
-        const u32 mlen = L.mid_b - L.mid_a;
-        if (L.mid_fwd) p = rput_bytes(p, S.mid, mlen);
-        else {
-            u32 t = 0;   // output order is the reverse token order: first text token is written last
-            while (t < mlen) {
-                u32 e = t;
-                while (S.mid[e] <= '9') ++e;   // the op letter ends the token
-                for (u32 k = e + 1; k-- > t;) *--p = S.mid[k];
-                t = e + 1;
-            }
+    const u32 mlen = L.mid_b > L.mid_a ? L.mid_b - L.mid_a : 0u;
+    u8* const pmid = p - mlen;   // FLAT_MID: written last, when the other fields are no longer live
+    if (FLAT_MID || mlen == 0) p = pmid;
+    else if (L.mid_fwd) p = rput_bytes(p, S.mid, mlen);
+    else {
+        u32 t = 0;   // output order is the reverse token order: first text token is written last
+        while (t < mlen) {
+            u32 e = t;
+            while (S.mid[e] <= '9') ++e;   // the op letter ends the token
+            for (u32 k = e + 1; k-- > t;) *--p = S.mid[k];
+            t = e + 1;
         }
     }
     if (!L.rev) { if (L.codeS) { *--p = L.codeS; p = rput_u32(p, L.lenS); } }
@@ -304,6 +341,7 @@ __device__ __forceinline__ u8* write_line(u8* pend, const LineSrc& S, const Line
     p = rput_u32(p, L.q0); *--p = '\t';
     p = rput_i32(p, R.qlen); *--p = '\t';
     p = rput_bytes(p, S.qname, R.qn_b);
+    if (FLAT_MID) put_tokens(pmid, S.mid, mlen, !L.mid_fwd);
     return p;
 }
 
@@ -817,12 +855,22 @@ __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.
 #endif
 
 constexpr int kEThreads = 256;
-constexpr u32 kEOutCap = 5120;     // staged PAF bytes per warp
 #ifndef G2P_EMIT_TEXT_CAP
 #define G2P_EMIT_TEXT_CAP 4096
 #endif
-constexpr u32 kETextCap = G2P_EMIT_TEXT_CAP;    // staged GAF bytes per warp (the records its 32 lines come from); 0: read the text from global
-constexpr size_t kEmitSmem = (size_t)(kEThreads / 32) * (kEOutCap + 16 + kETextCap + 32);
+// Staging buffers per warp: PAF bytes (out) and GAF bytes (text: the records its 32 lines come from; 0: read the
+// text from global).  Dense runs (k_par / k_long lines of long records) take 5 kB + 4 kB, 3 CTAs per SM.  The
+// line-map instantiation only stages one warp's run of k_rec lines -- 32 lines of ~130 bytes from ~14 records of
+// at most kSLimit bytes: ~4.3 kB of PAF from ~2 kB of GAF in short-read input -- and takes direct stores or global
+// reads for a run that does not fit, so its buffers are sized for 4 CTAs of 256 threads per SM (32 warps).
+template <bool DENSE> struct EmitCap {
+    static constexpr u32 out = DENSE ? 5120u : 4608u;
+    static constexpr u32 text = DENSE || G2P_EMIT_TEXT_CAP == 0 ? (u32)G2P_EMIT_TEXT_CAP : 2496u;
+    static constexpr size_t smem = (size_t)(kEThreads / 32) * (out + 16 + text + 32);
+};
+constexpr size_t kEmitSmem = EmitCap<true>::smem;        // dense runs (also enough for the line-map instantiation)
+constexpr size_t kEmitSmemMap = EmitCap<false>::smem;
+static_assert(4 * (kEmitSmemMap + 64 + 1024) <= 228 * 1024, "4 CTAs of the line-map instantiation per SM");
 
 // What k_emit_lines needs to start all its loads at once for a line of a k_short record.
 struct __align__(16) LineMapEnt {
@@ -850,6 +898,7 @@ struct EmitArgs {
 template <bool DENSE>
 __global__ void __launch_bounds__(kEThreads, DENSE ? 3 : 4) k_emit_lines(const EmitArgs a) {
     G2P_DYN_SMEM(smem);
+    constexpr u32 kEOutCap = EmitCap<DENSE>::out, kETextCap = EmitCap<DENSE>::text;
     const u32 FULL = 0xffffffffu;
     const u32 lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     u8* sm = smem + (size_t)warp * (kEOutCap + 16 + kETextCap + 32);
@@ -995,7 +1044,7 @@ __global__ void __launch_bounds__(kEThreads, DENSE ? 3 : 4) k_emit_lines(const E
     const u64 o1 = __shfl_sync(FULL, end, last);
     // short records: one run that fits the buffer (32 lines of ~130 bytes); anything else goes straight to global
     if (__any_sync(FULL, gap) || holes || (!DENSE && (o1 - __shfl_sync(FULL, o, first)) + 15u > kEOutCap)) {
-        if (valid) write_line(a.out + o + d.len, parts ? PS : line_src(rt, R, L), R, L);
+        if (valid) write_line<!DENSE>(a.out + o + d.len, parts ? PS : line_src(rt, R, L), R, L);
         return;
     }
     // The warp's lines are one contiguous run of the output.  It goes through the staging buffer in
@@ -1009,7 +1058,7 @@ __global__ void __launch_bounds__(kEThreads, DENSE ? 3 : 4) k_emit_lines(const E
         const bool fits = DENSE ? ((todo >> lane) & 1u) != 0 && (end - ob) + pad <= kEOutCap : valid;
         const u32 in = DENSE ? __ballot_sync(FULL, fits) : vmask;   // a prefix of `todo`: the lines are in output order
         if (DENSE && in == 0) {   // one line longer than the buffer
-            if ((int)lane == f) write_line(a.out + o + d.len, parts ? PS : line_src(rt, R, L), R, L);
+            if ((int)lane == f) write_line<!DENSE>(a.out + o + d.len, parts ? PS : line_src(rt, R, L), R, L);
             todo &= todo - 1u;
             continue;
         }
@@ -1017,9 +1066,9 @@ __global__ void __launch_bounds__(kEThreads, DENSE ? 3 : 4) k_emit_lines(const E
         if (fits) {
             // two instantiations so that the common one (staged lines, staged text) works on pointers the
             // compiler can prove to be shared memory: LDS / STS instead of generic 64-bit LD / ST
-            if (text_staged) write_line(sm + pad + (u32)(o - ob) + d.len, line_src(sm_text + (rs - A), R, L), R, L);
-            else if (DENSE && parts) write_line(sm + pad + (u32)(o - ob) + d.len, PS, R, L);
-            else write_line(sm + pad + (u32)(o - ob) + d.len, line_src(a.gaf + rs, R, L), R, L);   // long records: text from global
+            if (text_staged) write_line<!DENSE>(sm + pad + (u32)(o - ob) + d.len, line_src(sm_text + (rs - A), R, L), R, L);
+            else if (DENSE && parts) write_line<!DENSE>(sm + pad + (u32)(o - ob) + d.len, PS, R, L);
+            else write_line<!DENSE>(sm + pad + (u32)(o - ob) + d.len, line_src(a.gaf + rs, R, L), R, L);   // long records: text from global
         }
         const u32 total = pad + (u32)(oe - ob);
         u8* gb = a.out + (ob - pad);
